@@ -3,7 +3,7 @@
 bench.py -- rays/sec of the pixelNeRF render hot path on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c4] [--scaling weak|strong]
-                  [--impl ours|reference|reference-gpu|torch-eager]
+                  [--impl ours|reference|reference-gpu|torch-eager] [--dump-outputs DIR]
   torchrun --nproc-per-node N ... bench.py --gpus N ...   (one rank per GPU, NCCL)
 
 A "step" renders one batch of synthetic rays (coarse + fine pass) of a BASELINE.json workload:
@@ -21,7 +21,11 @@ broadcast from rank 0 once (NCCL) and rendered pixels are gathered to rank 0 eve
 The line also carries a `parity` block: the benchmarked model + frame, 256 rays with injected noise, CUDA vs the CPU
 oracle (outside the timed region).
 
-`--impl reference` times the UNMODIFIED reference (baseline/_ref, installed by scripts/install_ref.py; falls back to the
+`--dump-outputs DIR` writes the rgb / depth of the last timed step, so that two builds run with the same arguments
+(hence the same seeded scene, rays and sample noise) can be compared output for output.  Nothing is written into the
+source tree: no bytecode either, so the tree may be read-only.
+
+`--impl reference` times the UNMODIFIED reference (oracle/_ref, installed by build(); falls back to the
 oracle port when absent) on the HOST CPU cores through its own public API, on a bounded sample of the same workload;
 `--impl reference-gpu` runs the same unmodified reference eagerly on the B200(s) (fp32, TF32 off; DataParallel at N>1) --
 the denominator of north_star's ">= 10x the reference's own 1xGPU PyTorch rays/sec".
@@ -38,6 +42,7 @@ import time
 
 import torch
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "pixel-nerf_b200")
 SRC = os.path.join(PKG, "src")
@@ -231,6 +236,24 @@ def parity_block(net, renderer, cfg, rays_dev, n=256):
             "oracle_seconds": t_oracle}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> (1, rays, ...) tensor, written as out_dir/<name>.npy in float32.  Above DUMP_LIMIT_BYTES in all,
+    a fixed, seeded sample of rays (the same rays for every array, in ray order) is written instead."""
+    import numpy as np
+    n = next(iter(arrays.values())).shape[1]
+    per_ray = sum(t[0, :1].numel() * 4 for t in arrays.values())
+    keep = None
+    if n * per_ray > DUMP_LIMIT_BYTES:
+        keep = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_LIMIT_BYTES // per_ray].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t if keep is None else t[:, keep]).numpy())
+
+
 def run_ours(args):
     if SRC not in sys.path:
         sys.path.insert(0, SRC)
@@ -292,20 +315,21 @@ def run_ours(args):
             host_dep.copy_(depth, non_blocking=True)
 
     def timed(fn, steps):
+        """(device ms of `steps` calls of fn, what the last call returned)"""
         if dist is not None:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=device)
         if dist is not None:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), last
 
     warm = max(args.warmup, 3)
     for _ in range(warm):
@@ -317,7 +341,7 @@ def run_ours(args):
         sampler.start()
     launches0 = pn.launch_count()
     pn.profile_begin()
-    ms_total = timed(step_resident, args.steps)
+    ms_total, (last_rgb, last_depth) = timed(step_resident, args.steps)
     kern_ms, kern_launches = pn.profile_end()
     if os.environ.get("PNR_TC_COUNTERS"):
         names = ["mma_total", "mma_wait_a_first_chunk", "mma_wait_b", "mma_wait_bpeer", "unused4", "unused5",
@@ -326,8 +350,10 @@ def run_ours(args):
     launches = pn.launch_count() - launches0
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     sampler.stop_flag = True
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rgb": last_rgb, "depth": last_depth})
 
     value = total * args.steps / (ms_total / 1e3)
     e2e_value = total * args.steps / (ms_e2e / 1e3)
@@ -393,10 +419,10 @@ def run_ours(args):
 
 
 # ------------------------------------------------------------------------------------------
-# reference arms: the UNMODIFIED reference through its own public API (baseline/_ref)
+# reference arms: the UNMODIFIED reference through its own public API (oracle/_ref)
 # ------------------------------------------------------------------------------------------
 def reference_root():
-    for root in (os.environ.get("PIXELNERF_REF"), os.path.join(ROOT, "baseline", "_ref")):
+    for root in (os.environ.get("PIXELNERF_REF"), os.path.join(ROOT, "oracle", "_ref")):
         if root and os.path.isdir(os.path.join(root, "src", "render")):
             return root
     return None
@@ -404,7 +430,7 @@ def reference_root():
 
 def build_reference_scene(workload, device):
     """The reference's PixelNeRFNet + NeRFRenderer + bind_parallel, weights and scene of the workload; returns
-    (net, renderer) or None when baseline/_ref is absent."""
+    (net, renderer) or None when oracle/_ref is absent."""
     root = reference_root()
     if root is None:
         return None
@@ -457,7 +483,7 @@ def cpu_arm(workload):
         def render(rays):
             with torch.no_grad():
                 return render_par(rays)
-        kind, what = "reference", "unmodified reference (baseline/_ref) NeRFRenderer.bind_parallel(net)(rays), torch CPU fp32"
+        kind, what = "reference", "unmodified reference (oracle/_ref) NeRFRenderer.bind_parallel(net)(rays), torch CPU fp32"
     else:
         oracle = _load("pnr_oracle", os.path.join(ROOT, "oracle", "pnr_oracle.py"))
         src, _, focal, c = synth.make_cameras(cfg)
@@ -470,7 +496,7 @@ def cpu_arm(workload):
             with torch.no_grad():
                 return oracle.render(rays, noise, state, latent, wc, wf, cfg["NS"], cfg["n_coarse"], cfg["n_fine"],
                                      cfg["n_fine_depth"], white_bkgd=cfg["white_bkgd"], eval_batch_size=50000)
-        kind, what = "port", "oracle/pnr_oracle.py (baseline/_ref absent), torch CPU fp32"
+        kind, what = "port", "oracle/pnr_oracle.py (oracle/_ref absent), torch CPU fp32"
     ncpu = os.cpu_count() or 1
     cands = sorted({t for t in (8, 16, 32, 64, 128, ncpu) if t <= ncpu})
     probe_rays = synth.make_rays(cfg, 64)[None]
@@ -541,7 +567,7 @@ def run_reference_gpu(args):
     wl = WORKLOADS[args.workload]
     cfg = synth.CONFIGS[args.workload]
     if reference_root() is None:
-        print(json.dumps({"impl": "reference-gpu", "unavailable": "baseline/_ref not installed (scripts/install_ref.py)"}))
+        print(json.dumps({"impl": "reference-gpu", "unavailable": "oracle/_ref not installed (build() with a reference checkout)"}))
         return
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
@@ -578,7 +604,7 @@ def run_reference_gpu(args):
                       "dtype": "f32 (TF32 off)", "data": "synthetic",
                       "config": {"workload": wl["text"], "rays_per_step": total, "ray_batch_size": 50000,
                                  "parallelism": "single GPU" if args.gpus == 1 else f"nn.DataParallel(dim=1) x{args.gpus}",
-                                 "note": "unmodified reference (baseline/_ref), PyTorch eager"}}))
+                                 "note": "unmodified reference (oracle/_ref), PyTorch eager"}}))
 
 
 def run_torch_eager(args):
@@ -635,7 +661,14 @@ if __name__ == "__main__":
     ap.add_argument("--cpu-rays", type=int, default=0, help="rays per CPU-reference pass (default per workload)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rgb / depth the last timed step rendered as DIR/<name>.npy (float32, at most 64 MB "
+                         "in all: a fixed sample of rays above that); the same arguments give the same inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours renders")
     if a.impl == "reference":
         run_reference(a)
     elif a.impl == "reference-gpu":

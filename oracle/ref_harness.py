@@ -1,13 +1,13 @@
 """
 ORACLE TOOLING -- TEST INFRASTRUCTURE, NOT PRODUCT CODE.
 
-Imports the UNMODIFIED reference (sxyu/pixel-nerf) from /root/reference/src (or
-$PIXELNERF_REF) on CPU so that `make_golden.py` can generate golden vectors and the
+Imports the UNMODIFIED reference (sxyu/pixel-nerf) from $PIXELNERF_REF/src, else from the
+copy build() installs in oracle/_ref/src, on CPU so that `make_golden.py` can generate golden vectors and the
 restatement in `pnr_oracle.py` can be validated against the real thing.  The reference
 needs two pure-Python packages that are not installed here (`dotmap`, `pyhocon`); tiny
 stand-ins are injected into sys.modules ONLY for that import -- no reference source is
-copied or changed.  This module cannot run on the GPU box (no /root/reference there) and
-nothing in tests -m gpu / smoke() / bench.py uses it.
+copied or changed.  The tests do not use it: they compare with golden data it helped write.
+bench.py's reference timing arms do, when oracle/_ref is installed.
 """
 import os
 import sys
@@ -19,12 +19,12 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _find_ref():
-    """$PIXELNERF_REF, else /root/reference (this container), else baseline/_ref (the copy scripts/install_ref.py ships
-    to the GPU box for the timing arms of bench.py)."""
-    for root in (os.environ.get("PIXELNERF_REF"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")):
+    """$PIXELNERF_REF, else oracle/_ref (oracle/install_ref.py, run by build())."""
+    installed = os.path.join(_REPO, "oracle", "_ref")
+    for root in (os.environ.get("PIXELNERF_REF"), installed):
         if root and os.path.isdir(os.path.join(root, "src")):
             return root
-    return "/root/reference"
+    return installed
 
 
 REF_ROOT = _find_ref()

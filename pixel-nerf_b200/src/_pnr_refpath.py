@@ -5,7 +5,7 @@ This package replaces the render hot path only.  The reference's callers (`train
 `eval/gen_video.py:11-16`) also import `data.get_split_dataset`, `model.loss`, `util.cmap`, ... from the same `src/`
 directory; those names resolve to the reference's own, unmodified files, located through
 
-    $PIXELNERF_REF  ->  <repo>/baseline/_ref  ->  /root/reference        (first that has a `src/` directory)
+    $PIXELNERF_REF  ->  <repo>/oracle/_ref (installed there by build())        (first that has a `src/` directory)
 
 Nothing of the reference is copied into this package; without a reference checkout those names raise ImportError /
 AttributeError naming this module, and the hot-path classes still work.
@@ -19,7 +19,7 @@ _REPO = os.path.dirname(os.path.dirname(_HERE))
 def candidates():
     env = os.environ.get("PIXELNERF_REF")
     out = [env] if env else []
-    out += [os.path.join(_REPO, "baseline", "_ref"), "/root/reference"]
+    out.append(os.path.join(_REPO, "oracle", "_ref"))
     return out
 
 

@@ -6,7 +6,7 @@ with want_weights=True, MSE coarse + MSE fine, backward through MLPs and the enc
     python scripts/bench_train.py --mode render     # the package default: pnr_render + pnr_render_backward in one node
     python scripts/bench_train.py --mode field      # PNR_FUSED_BACKWARD=1: torch renderer, fused field fwd + pnr_field_backward
     python scripts/bench_train.py --mode torch      # PNR_FUSED_BACKWARD=0: composed-torch grad path of this package
-    python scripts/bench_train.py --mode reference  # the UNMODIFIED reference (baseline/_ref), same step, same GPU
+    python scripts/bench_train.py --mode reference  # the UNMODIFIED reference (oracle/_ref), same step, same GPU
 
 `--device cpu --tiny` checks the script itself (torch mode)."""
 import argparse
@@ -40,7 +40,7 @@ def main():
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
     if a.mode == "reference":
-        # the reference's own classes (packages `model` / `render` / `util` of baseline/_ref instead of this repo's)
+        # the reference's own classes (packages `model` / `render` / `util` of oracle/_ref instead of this repo's)
         sys.path.remove(os.path.join(ROOT, "pixel-nerf_b200", "src"))
         sys.path.insert(0, os.path.join(ROOT, "oracle"))
         import ref_harness as rh

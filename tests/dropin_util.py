@@ -22,7 +22,7 @@ install_ref = _load("pnr_install_ref", os.path.join(ROOT, "scripts", "install_re
 
 
 def reference_root():
-    """The reference checkout for tests: /root/reference here, baseline/_ref on the GPU box; None if neither."""
+    """The reference checkout for tests: $PIXELNERF_REF, else the copy build() installs in oracle/_ref; None if neither."""
     return install_ref.find_reference()
 
 

@@ -1,6 +1,6 @@
 """The reference's UNMODIFIED eval/gen_video.py and train/train.py, run end to end on the GPU against this package through
 the overlay tree (scripts/install_ref.py): synthetic SRN-format dataset on disk, reference conf/exp/srn.conf with the
-ImageNet download switched off.  On the GPU box the reference comes from baseline/_ref."""
+ImageNet download switched off.  The reference comes from oracle/_ref (installed by build())."""
 import glob
 import os
 
@@ -11,7 +11,7 @@ import torch
 import dropin_util as du
 
 pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(du.reference_root() is None, reason="no reference checkout (baseline/_ref)")]
+              pytest.mark.skipif(du.reference_root() is None, reason="no reference checkout (oracle/_ref: build() with one present, or PIXELNERF_REF)")]
 
 
 def test_gen_video_main_runs_unmodified(tmp_path):

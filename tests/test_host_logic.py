@@ -1,5 +1,6 @@
 """Host-side logic on CPU: HOCON reader, conf files, model/renderer construction, state_dict
 compatibility, unsupported-flag errors, schedule, DotMap, no-CPU-fallback guard."""
+import json
 import os
 import sys
 
@@ -13,6 +14,7 @@ sys.path.insert(0, os.path.join(PKG, "src"))
 from util import hocon  # noqa: E402
 import golden_util as gu  # noqa: E402
 import gpu_util  # noqa: E402
+import ref_recipes  # noqa: E402
 
 
 def test_hocon_subset():
@@ -45,32 +47,15 @@ def test_conf_files_resolve_includes(name):
                                            "multi_obj": "multi_obj"}[name]
 
 
-def _flatten(c, prefix=""):
-    out = {}
-    for k in c.keys():
-        v = c[k]
-        if hasattr(v, "keys"):
-            out.update(_flatten(v, prefix + k + "."))
-        else:
-            out[prefix + k] = v
-    return out
-
-
 def test_shipped_confs_equal_the_reference_confs():
     """Every exp conf and expconf.conf of this package parses to the same tree as the reference's own file (read with
-    the same in-repo HOCON reader; the reference's files are the schema)."""
-    ref = None
-    for root in (os.environ.get("PIXELNERF_REF"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if root and os.path.isdir(os.path.join(root, "conf", "exp")):
-            ref = root
-            break
-    if ref is None:
-        pytest.skip("no reference checkout")
-    for name in sorted(os.listdir(os.path.join(ref, "conf", "exp"))):
-        ours = hocon.parse_file(os.path.join(PKG, "conf", "exp", name))
-        theirs = hocon.parse_file(os.path.join(ref, "conf", "exp", name))
-        assert _flatten(ours) == _flatten(theirs), name
-    assert _flatten(hocon.parse_file(os.path.join(PKG, "expconf.conf"))) == _flatten(hocon.parse_file(os.path.join(ref, "expconf.conf")))
+    the same in-repo HOCON reader; the reference's files are the schema, stored parsed in tests/golden/ref_confs.json
+    by tests/ref_probe.py)."""
+    with open(os.path.join(gu.GOLD, "ref_confs.json")) as f:
+        theirs = json.load(f)
+    assert len(theirs) == 6 and "expconf.conf" in theirs
+    for name, tree in theirs.items():
+        assert ref_recipes.flatten(hocon.parse_file(os.path.join(PKG, name))) == tree, name
 
 
 def test_model_state_dict_keys_and_shapes():

@@ -1,31 +1,24 @@
-"""State producer and checkpoint compatibility against the UNMODIFIED reference (run in its own interpreter by
-tests/ref_probe.py):
+"""State producer and checkpoint compatibility against the UNMODIFIED reference, through the golden data that
+tests/ref_probe.py wrote by running it (tests/golden/ref_encoder.npz, ref_checkpoint.npz); the seeded recipes both
+share are in tests/ref_recipes.py:
 
   * a19: `SpatialEncoder.forward` / `PixelNeRFNet.encode` -- same state_dict, same images -> the same latent, camera
     state and `index()` values as the reference (src/model/encoder.py:111-164, src/model/models.py:89-144);
-  * f-4: a checkpoint written by the reference's own `save_weights` strict-loads here and gives the reference's field
-    values; a checkpoint written here strict-loads in the reference (src/model/models.py:268-316).
+  * f-4: a checkpoint as the reference's own `save_weights` writes it strict-loads here and gives the reference's field
+    values; a checkpoint written here has the names, order, shapes and values the reference's strict
+    `load_weights` needs (src/model/models.py:268-316).
 """
 import os
-import subprocess
-import sys
 
-import pytest
+import numpy as np
 import torch
 
-import dropin_util as du
+import golden_util as gu
 import gpu_util
+import ref_recipes
 
-PROBE = os.path.join(du.ROOT, "tests", "ref_probe.py")
-needs_ref = pytest.mark.skipif(du.reference_root() is None, reason="no reference checkout (/root/reference or baseline/_ref)")
-
-
-def probe(*argv):
-    env = dict(os.environ)
-    env["PIXELNERF_REF"] = du.reference_root()
-    r = subprocess.run([sys.executable, PROBE, *argv], env=env, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
-    return r.stdout
+ENC = np.load(os.path.join(gu.GOLD, "ref_encoder.npz"))
+CKPT = np.load(os.path.join(gu.GOLD, "ref_checkpoint.npz"))
 
 
 class Args:
@@ -33,53 +26,72 @@ class Args:
         self.checkpoints_path, self.name, self.resume = d, name, resume
 
 
-@needs_ref
-def test_encoder_and_encode_state_match_the_reference(tmp_path):
-    out = str(tmp_path / "enc.pt")
-    probe("encoder", out)
-    cases = torch.load(out)
+def assert_same_state(sd, keys, digests):
+    """Same names in the same order, and bit-identical tensors, as the reference's state_dict."""
+    assert list(sd.keys()) == keys.tolist()
+    bad = [k for k, d in zip(keys, digests) if not np.array_equal(ref_recipes.digest(sd[k]), d)]
+    assert not bad, f"tensors differ from the reference's: {bad[:5]}"
+
+
+def assert_sampled(t, z, prefix, seed, rel, mean_dims):
+    """|t - ref| <= rel * max|ref| on the stored sample of elements and on the per-channel means (ref_probe.sampled)."""
+    tol = rel * float(z[prefix + "_max"])
+    assert tuple(t.shape) == tuple(z[prefix + "_shape"]), prefix
+    idx = ref_recipes.sample_index(t.numel(), seed)
+    assert (t.reshape(-1)[idx] - torch.from_numpy(z[prefix + "_sample"])).abs().max() <= tol, prefix
+    assert (t.double().mean(mean_dims) - torch.from_numpy(z[prefix + "_mean"])).abs().max() <= tol, prefix
+
+
+def test_encoder_and_encode_state_match_the_reference():
     from model import make_model
-    for name, ref in cases.items():
-        net = make_model(gpu_util.model_conf(64, ref["use_first_pool"])).eval()
-        missing = net.load_state_dict(ref["state_dict"], strict=True)
-        assert not missing.missing_keys and not missing.unexpected_keys
+    for name, use_first_pool, (SB, NS, H, W) in ref_recipes.ENCODER_CASES:
+        g = lambda k: ENC[f"{name}/{k}"]
+        net = ref_recipes.encoder_net(make_model, gpu_util.model_conf, use_first_pool)
+        assert_same_state(net.state_dict(), g("sd_keys"), g("sd_digest"))
+        images, poses, focal, c = ref_recipes.scene(7, SB, NS, H, W)
+        assert np.array_equal(np.stack([ref_recipes.digest(t) for t in (images, poses, focal, c)]), g("inputs_digest"))
+        uv = ref_recipes.encoder_uv(SB, NS, H, W)
+        assert torch.equal(uv, torch.from_numpy(g("uv")))
         with torch.enable_grad():     # CPU tensors: the composed-torch path (encode() itself has no fused part)
-            net.encode(ref["images"], ref["poses"], ref["focal"], c=ref["c"])
-            idx = net.encoder.index(ref["uv"], None, net.image_shape)
-        lat = net.encoder.latent.detach()
-        assert lat.shape == ref["latent"].shape, name
-        assert (lat - ref["latent"]).abs().max() <= 1e-6 * ref["latent"].abs().max(), name
-        assert torch.equal(net.encoder.latent_scaling, ref["latent_scaling"])
-        assert torch.equal(net.poses, ref["poses_state"])
-        assert torch.equal(net.focal, ref["focal_state"]) and torch.equal(net.c, ref["c_state"])
-        assert torch.equal(net.image_shape, ref["image_shape"])
-        assert net.num_views_per_obj == ref["num_views_per_obj"]
-        assert (idx.detach() - ref["index"]).abs().max() <= 1e-5 * ref["index"].abs().max()
+            net.encode(images, poses, focal, c=c)
+            idx = net.encoder.index(uv, None, net.image_shape)
+        assert_sampled(net.encoder.latent.detach(), ENC, f"{name}/latent", 1, 1e-6, (2, 3))
+        assert torch.equal(net.encoder.latent_scaling, torch.from_numpy(g("latent_scaling")))
+        assert torch.equal(net.poses, torch.from_numpy(g("poses_state")))
+        assert torch.equal(net.focal, torch.from_numpy(g("focal_state")))
+        assert torch.equal(net.c, torch.from_numpy(g("c_state")))
+        assert torch.equal(net.image_shape, torch.from_numpy(g("image_shape")))
+        assert net.num_views_per_obj == int(g("num_views_per_obj"))
+        assert_sampled(idx.detach(), ENC, f"{name}/index", 2, 1e-5, (1,))
 
 
-@needs_ref
 def test_checkpoints_round_trip_with_the_reference(tmp_path):
-    d = str(tmp_path)
-    probe("checkpoint", d)
-    assert os.path.exists(os.path.join(d, "probe", "pixel_nerf_latest"))
-    assert os.path.exists(os.path.join(d, "probe", "pixel_nerf_backup"))
-    io = torch.load(os.path.join(d, "probe_io.pt"))
     from model import make_model
+    d = str(tmp_path)
+    # the checkpoint the reference's save_weights wrote: torch.save(state_dict) at <checkpoints>/<name>/pixel_nerf_latest
+    src = ref_recipes.checkpoint_net(make_model, gpu_util.model_conf).state_dict()
+    assert_same_state(src, CKPT["sd_keys"], CKPT["sd_digest"])
+    os.makedirs(os.path.join(d, "probe"))
+    torch.save(src, os.path.join(d, "probe", "pixel_nerf_latest"))
     net = make_model(gpu_util.model_conf(512, True)).eval()
-    assert list(net.state_dict().keys()) == io["keys"]            # same names, same order
+    before = net.mlp_coarse.lin_in.weight.clone()
     assert net.load_weights(Args(d, "probe"), strict=True) is net
+    assert not torch.equal(before, net.mlp_coarse.lin_in.weight), "checkpoint was not loaded"
+    images, poses, focal, c = ref_recipes.scene(5, 1, 2, 32, 32)
+    assert np.array_equal(np.stack([ref_recipes.digest(t) for t in (images, poses, focal, c)]), CKPT["inputs_digest"])
+    xyz, dirs = torch.from_numpy(CKPT["xyz"]), torch.from_numpy(CKPT["dirs"])
     with torch.enable_grad():                                      # CPU: composed-torch field
-        net.encode(io["images"], io["poses"], io["focal"], c=io["c"])
-        oc = net(io["xyz"].requires_grad_(True), coarse=True, viewdirs=io["dirs"]).detach()
-        of = net(io["xyz"], coarse=False, viewdirs=io["dirs"]).detach()
-    assert (oc - io["out_coarse"]).abs().max() < 1e-5
-    assert (of - io["out_fine"]).abs().max() < 1e-5
-    # and back: our save_weights -> the reference's load_weights(strict=True) -> its forward gives the same values
+        net.encode(images, poses, focal, c=c)
+        oc = net(xyz.requires_grad_(True), coarse=True, viewdirs=dirs).detach()
+        of = net(xyz, coarse=False, viewdirs=dirs).detach()
+    assert (oc - torch.from_numpy(CKPT["out_coarse"])).abs().max() < 1e-5
+    assert (of - torch.from_numpy(CKPT["out_fine"])).abs().max() < 1e-5
+    # and back: our save_weights writes the files the reference's writes, and what the reference's
+    # load_weights(strict=True) reads from them is the state it computed out_coarse / out_fine with
     os.makedirs(os.path.join(d, "ours"), exist_ok=True)
     net.save_weights(Args(d, "ours"))
     net.save_weights(Args(d, "ours"))
-    assert os.path.exists(os.path.join(d, "ours", "pixel_nerf_backup"))
-    out = probe("load", d)
-    assert float(out.strip().split("MAXDIFF")[-1]) < 1e-6
+    assert sorted(os.listdir(os.path.join(d, "ours"))) == CKPT["files"].tolist()
+    assert_same_state(torch.load(os.path.join(d, "ours", "pixel_nerf_latest")), CKPT["sd_keys"], CKPT["sd_digest"])
     # opt_init semantics (models.py:276-283): no resume + opt_init -> nothing is loaded, returns None
     assert net.load_weights(Args(d, "probe", resume=False), opt_init=True) is None
